@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA path through the C ABI)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's own CPU implementation
+    python bench.py --gpus 1 --dump-outputs DIR              # also writes the last timed step's outputs (see dump_outputs)
 
 Workload (BASELINE.json configs[2], the configuration the metric's "1/2/4/8 B200" is quoted on): ONE synthetic 16 GB
 FASTQ file image of 100 bp reads with N runs and a 41-symbol quality alphabet.  Strong scaling with the reference's own
@@ -42,6 +43,8 @@ WORKLOADS = {  # name -> description
     "var50_205": "variable-length 50-205 bp reads, 17-field titles, skewed quality (configs[4] shape, in-domain cap)",
 }
 SEGMENT_MB = 1000
+PORT_SAMPLE_BYTES = 64_000_000  # the oracle port is a scalar single-core loop: a larger sample only costs time
+DUMP_BYTES = 64_000_000  # most bytes --dump-outputs writes, all files together
 
 
 def parse_args():
@@ -57,7 +60,13 @@ def parse_args():
     ap.add_argument("--driver-mb", type=int, default=8000, help="file size of the file-to-file driver leg (0: skip it)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-shapes", action="store_true", help="skip the 1 GB kernel-only probes of the other named shapes (N = 1 only)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed kernel-only step returned to DIR/*.npy (see dump_outputs)")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
+    return a
 
 
 class ClockSampler:
@@ -151,6 +160,35 @@ def record_stats(data):
     return nrec, title, seq
 
 
+def whole_records(data, n):
+    """data[:n] cut back to the end of its last complete four-line record."""
+    nl = np.flatnonzero(data[:n] == 10)
+    return data[:int(nl[(nl.size // 4) * 4 - 1]) + 1]
+
+
+def dump_outputs(path, descs, res, out, budget, prefix=""):
+    """Writes what one compress_resident + download returned, so that two builds can be compared output for output:
+      descs.npy           float64 [n_subblocks, 14]: every descriptor field in SubblockDesc order (sec_len as four columns)
+      result.npy          float64 [6]: n_subblocks, n_batches, bytes_in, bytes_out, out_used, wr_overlap
+      payload_sample.npy  float32: payload bytes of the payloads laid end to end (the alignment gaps between them are not
+                          outputs) -- all of them if they fit `budget`, else those at the sorted positions
+                          np.random.default_rng(0).integers(0, bytes_out, n)
+    Times and launch counts are left out: they are how the call ran, not what it computed."""
+    rows = np.array([[d.win_off, d.win_len, d.rec_start, d.overlap, d.n_records, d.warnings, d.bytes_consumed, *d.sec_len,
+                      d.out_off, d.out_len, d.status] for d in descs], np.float64).reshape(-1, 14)
+    result = np.array([res.n_subblocks, res.n_batches, res.bytes_in, res.bytes_out, res.out_used, res.wr_overlap], np.float64)
+    off, ln = rows[:, 11].astype(np.int64), rows[:, 12].astype(np.int64)
+    ends = np.cumsum(ln)
+    total = int(ends[-1]) if ln.size else 0
+    n = max(0, min(total, (budget - rows.nbytes - result.nbytes - 3 * 128) // 4))  # 128: an .npy header
+    pos = np.arange(total) if n == total else np.sort(np.random.default_rng(0).integers(0, total, n))
+    i = np.searchsorted(ends, pos, side="right")
+    sample = out[off[i] + pos - (ends[i] - ln[i])].astype(np.float32)
+    os.makedirs(path, exist_ok=True)
+    for name, arr in (("descs", rows), ("result", result), ("payload_sample", sample)):
+        np.save(os.path.join(path, prefix + name + ".npy"), arr)
+
+
 def host_cores():
     try:
         return len(os.sched_getaffinity(0))
@@ -165,10 +203,8 @@ def run_reference_sample(data, sample_bytes, tmpdir="/dev/shm"):
     Falls back to the oracle port (one core) when the reference binary is not there.
     -> dict(value GB/s, cores, kind, sample, seconds)"""
     from oracle import phy_oracle as O
-    n = min(sample_bytes, data.size)
-    nl = np.flatnonzero(data[:n] == 10)
-    cut = int(nl[(nl.size // 4) * 4 - 1]) + 1  # whole records only
-    sample = data[:cut]
+    sample = whole_records(data, sample_bytes)
+    cut = sample.size
     cores = host_cores()
     if O.have_reference():
         npr = max(2, min(cores, 64))
@@ -189,7 +225,7 @@ def run_reference_sample(data, sample_bytes, tmpdir="/dev/shm"):
                     sample=f"first {cut} bytes of the file image, unmodified reference, np={npr} x threads=1 over the fork-based MPI stand-in, "
                            f"tmpfs I/O included (max COMP_TIME {secs:.3f}s, wall {wall:.3f}s)")
     O.build()
-    small = sample[: min(cut, 64_000_000)]
+    small = whole_records(sample, PORT_SAMPLE_BYTES)  # a record cut short would be malformed input to the port
     t = time.perf_counter()
     O.compress_rank(small, 1, 0)
     secs = time.perf_counter() - t
@@ -328,6 +364,9 @@ def main():
     total_in = sum_over_ranks(float(bytes_in))
     total_out = sum_over_ranks(float(bytes_out))
     value = total_in / (ms_per_step * 1e-3) / 1e9
+    if a.dump_outputs:  # the payloads of the last timed step are still in device memory; pin_out is free until the e2e leg
+        ctx.download(pin_out.array)
+        dump_outputs(a.dump_outputs, descs, res, pin_out.array, DUMP_BYTES // world, f"rank{rank}_" if world > 1 else "")
 
     # ---- end to end from pinned host memory ---------------------------------------------------------------------
     # a second context with small batches: upload of batch b+1, kernels of batch b and download of batch b-1 overlap

@@ -1,11 +1,27 @@
 """Shared helpers of the GPU parity tests: run the CUDA path through the C ABI and diff it against the
 oracle, reporting the first differing section / byte so that one GPU run says as much as possible."""
+import hashlib
+import json
+import os
+
 import numpy as np
 
 from oracle import phy_oracle as O
 from phyngsc_b200 import api, synth
 
 SEC = ["info", "title", "quality", "dna"]
+REF_DIGESTS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_digests.json")
+
+
+def digest(b):
+    """Short content digest of one payload or block (64 bits of SHA-256)."""
+    return hashlib.sha256(b).hexdigest()[:16]
+
+
+def ref_digests(key):
+    """Stored stand-in for a compiled-reference run (tests/golden/make_reference_digests.py)."""
+    with open(REF_DIGESTS) as f:
+        return json.load(f)["cases"][key]
 
 
 def first_diff(a, b):
