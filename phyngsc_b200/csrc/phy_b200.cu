@@ -29,48 +29,107 @@ using namespace phy;
 static_assert(sizeof(phy_subblock_desc) == 72, "phy_subblock_desc layout is part of the ABI");
 static_assert(sizeof(phy_region_params) == 40, "phy_region_params layout is part of the ABI");
 
+/* Owning handles of a context's CUDA resources.  Each is complete or empty, never half made, and its destructor releases
+ * it: phy_ctx_destroy (and a failed ctx_init) only has to delete the context. */
+template <class T, bool Pinned> struct Buf { /* `cap` bytes of device memory, or of pinned host memory */
+  T *p = nullptr;
+  u64 cap = 0;
+  Buf() = default;
+  Buf(const Buf &) = delete;
+  Buf &operator=(const Buf &) = delete;
+  ~Buf() { release(); }
+  operator T *() const { return p; }
+  T *operator->() const { return p; }
+  void swap(Buf &o) { std::swap(p, o.p); std::swap(cap, o.cap); }
+  void release() {
+    if (p) { if (Pinned) cudaFreeHost(p); else cudaFree(p); }
+    p = nullptr; cap = 0;
+  }
+  /* At least `bytes`.  Growing frees the old buffer first (never two at a time) and leaves the buffer empty if it fails;
+   * `zero` clears a new buffer. */
+  cudaError_t ensure(u64 bytes, bool zero = false) {
+    if (cap >= bytes) return cudaSuccess;
+    release();
+    void *q = nullptr;
+    cudaError_t e = Pinned ? cudaHostAlloc(&q, bytes, cudaHostAllocDefault) : cudaMalloc(&q, bytes);
+    if (e != cudaSuccess) return e;
+    p = (T *)q; cap = bytes;
+    if (zero && (e = cudaMemset(p, 0, bytes)) != cudaSuccess) release();
+    return e;
+  }
+};
+template <class T> using DevBuf = Buf<T, false>;
+template <class T> using PinBuf = Buf<T, true>;
+
+static cudaError_t create(cudaStream_t *s, int priority) { return cudaStreamCreateWithPriority(s, cudaStreamNonBlocking, priority); }
+static cudaError_t create(cudaEvent_t *e, unsigned flags) { return cudaEventCreateWithFlags(e, flags); }
+static void destroy(cudaStream_t s) { cudaStreamDestroy(s); }
+static void destroy(cudaEvent_t e) { cudaEventDestroy(e); }
+template <class H, class Arg> struct Handle { /* a stream (ensure(priority)) or an event (ensure(flags)) */
+  H h = nullptr;
+  Handle() = default;
+  Handle(const Handle &) = delete;
+  Handle &operator=(const Handle &) = delete;
+  ~Handle() { if (h) destroy(h); }
+  operator H() const { return h; }
+  cudaError_t ensure(Arg a) {
+    if (h) return cudaSuccess;
+    H x = nullptr;
+    cudaError_t e = create(&x, a);
+    if (e == cudaSuccess) h = x;
+    return e;
+  }
+};
+using Stream = Handle<cudaStream_t, int>;
+using Event = Handle<cudaEvent_t, unsigned>;
+
+/* pinned staging of phy_compress_stream */
+static const u64 RING_CHUNK = 16ull << 20;
+static const int RING_SLOTS = 8;
+static const int HOUT_SLOTS = 4; /* pinned payload slots: one being filled by the copy engine, the others with the emitter thread */
+static const int READERS = 6;    /* reader threads */
+
 struct phy_ctx {
   int device = 0;
-  cudaStream_t stream = nullptr;
-  /* subblock groups of a batch: own stream, header (device + pinned mirror) and events */
-  cudaStream_t gstream[GROUPS_MAX] = {}; cudaEvent_t ev_rb[GROUPS_MAX] = {}, ev_scan[GROUPS_MAX] = {}, ev_done[GROUPS_MAX] = {};
-  BatchHdr *hdr_g = nullptr, *h_hdr_g = nullptr;
-  cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+  int prio_hi = 0; /* the back part's streams outrank the front part's: a front part running ahead only fills gaps */
   u64 max_batch = 0; u32 max_sb = 0; u32 maxrec = 0; u32 arena_words = 0; u64 out_cap = 0; u32 slack = 0;
   u32 max_tiles = 0;
+  Stream stream, s_prefix;
+  Event ev_prefix;    /* the front part launched last is done */
+  Event ev_k0, ev_k1; /* begin and end of a walk's kernel leg (phy_region_result::kernel_ms) */
+  /* subblock groups of a batch: own stream, header (device + pinned mirror) and events */
+  Stream gstream[GROUPS_MAX]; Event ev_rb[GROUPS_MAX], ev_scan[GROUPS_MAX], ev_done[GROUPS_MAX];
+  DevBuf<BatchHdr> hdr_g; PinBuf<BatchHdr> h_hdr_g;
   /* device buffers */
-  u8 *in = nullptr; u32 *te = nullptr, *se = nullptr, *rstart = nullptr; u16 *kx = nullptr; u32 *qoff = nullptr, *doff = nullptr, *toff = nullptr, *chunk_first = nullptr, *chunk_last = nullptr;
-  u32 *tile_cnt = nullptr, *tile_off = nullptr; uint2 *nl_mask = nullptr;
-  u32 *blk_mask = nullptr, *tv = nullptr, *tc = nullptr, *tp = nullptr, *v0 = nullptr; u64 tv_cap = 0; /* parsed titles (k_stat1 -> k_stat2 / k_enc_title); tv / tp grow on demand */
-  PlanState *plan_state = nullptr; SbPlan *plans = nullptr; BatchHdr *hdr = nullptr;
-  SbAcc *acc = nullptr; SbClass *cls = nullptr; SbOut *sbout = nullptr; u32 *arena = nullptr; u8 *out = nullptr;
-  u32 *tmp = nullptr; u64 tmp_cap = 0; u64 *tmp_used = nullptr; /* temporary buffer of the single-walk encoder (words) */
+  DevBuf<u8> in; DevBuf<u32> te, se, rstart; DevBuf<u16> kx; DevBuf<u32> qoff, doff, toff, chunk_first, chunk_last;
+  DevBuf<u32> tile_cnt, tile_off; DevBuf<uint2> nl_mask;
+  DevBuf<u32> blk_mask, tv, tc, tp, v0; /* parsed titles (k_stat1 -> k_stat2 / k_enc_title); tv / tp / tc grow on demand */
+  DevBuf<PlanState> plan_state; DevBuf<SbPlan> plans; DevBuf<BatchHdr> hdr;
+  DevBuf<SbAcc> acc; DevBuf<SbClass> cls; DevBuf<SbOut> sbout; DevBuf<u32> arena; DevBuf<u8> out;
+  DevBuf<u32> tmp; DevBuf<u64> tmp_used; /* temporary buffer of the single-walk encoder (words) */
   /* second input / output buffers and copy streams of the pipelined region call (allocated on first use) */
-  u8 *in2 = nullptr, *out2 = nullptr;
-  cudaStream_t s_in = nullptr, s_out = nullptr;
-  cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_c[2] = {nullptr, nullptr}, ev_out[2] = {nullptr, nullptr};
-  cudaEvent_t ev_h0[2] = {nullptr, nullptr}, ev_d0[2] = {nullptr, nullptr};
-  u8 *h_nl = nullptr;
+  DevBuf<u8> in2, out2;
+  Stream s_in, s_out;
+  Event ev_in[2], ev_c[2], ev_out[2], ev_h0[2], ev_d0[2];
   /* pinned host mirrors */
-  BatchHdr *h_hdr = nullptr; SbPlan *h_plans = nullptr; SbOut *h_sbout = nullptr; PlanState *h_state = nullptr;
+  PinBuf<BatchHdr> h_hdr; PinBuf<SbPlan> h_plans; PinBuf<SbOut> h_sbout; PinBuf<PlanState> h_state;
   /* Front part of a batch (record splitter + window plan) ahead of its back part: the front part writes the "next" set of its
    * outputs (record table, window plans, header, host mirrors); prefix_finish() swaps that set with the current one, which the
    * back part (every other kernel) reads.  So the front part of batch b + 1 can run beside the back part of batch b. */
-  struct PrefixSet { u32 *te = nullptr, *se = nullptr, *rstart = nullptr; SbPlan *plans = nullptr; BatchHdr *hdr = nullptr;
-                     BatchHdr *h_hdr = nullptr; SbPlan *h_plans = nullptr; PlanState *h_state = nullptr; } nxt;
+  struct PrefixSet { DevBuf<u32> te, se, rstart; DevBuf<SbPlan> plans; DevBuf<BatchHdr> hdr;
+                     PinBuf<BatchHdr> h_hdr; PinBuf<SbPlan> h_plans; PinBuf<PlanState> h_state; } nxt;
   struct BatchArgs { const u8 *in = nullptr; u32 len = 0, start_pos = 0; i64 batch_base = 0, region_len = 0; bool is_final = false; } cur_args, nxt_args;
-  cudaStream_t s_prefix = nullptr; cudaEvent_t ev_prefix = nullptr;
   int pi = 0; /* next profiling event of the batch */
   u32 launches = 0;
   u64 resident_len = 0, resident_out = 0;
-  u8 *ring = nullptr, *hout[4] = {nullptr, nullptr, nullptr, nullptr}; cudaEvent_t ev_ring[8] = {}, ev_hout[4] = {}; /* pinned staging of phy_compress_stream */
-  u8 *big_in = nullptr, *big_out = nullptr; u64 big_in_cap = 0, big_out_cap = 0; /* resident regions larger than one batch (phy_upload) */
+  PinBuf<u8> ring, hout[HOUT_SLOTS]; Event ev_ring[RING_SLOTS], ev_hout[HOUT_SLOTS]; /* pinned staging of phy_compress_stream */
+  DevBuf<u8> big_in, big_out; /* resident regions larger than one batch (phy_upload) */
   u32 last_S = 0;
   u32 qcode_hint = 0; /* longest quality code the previous batch saw */
   u32 nq_hint = 0, prev_groups = 0, prev_max_len = 0; /* quality alphabet size seen by the previous batch (sizes the packed tables' shared memory without a readback) */
   /* per-kernel timing (phy_profile): one event after every launch of run_batch */
   bool profile = false;
-  cudaEvent_t pev[NKERN + 1] = {};
+  Event pev[NKERN + 1];
   float pms[NKERN] = {};
   u32 pcount = 0;
   std::string err;
@@ -128,36 +187,7 @@ extern "C" void phy_host_free(void *p) { if (p) cudaFreeHost(p); }
 
 extern "C" void phy_ctx_destroy(phy_ctx *ctx) {
   if (!ctx) return;
-  cudaSetDevice(ctx->device);
-  void *dev[] = {ctx->in, ctx->te, ctx->se, ctx->rstart, ctx->kx, ctx->qoff, ctx->doff, ctx->toff, ctx->chunk_first, ctx->chunk_last, ctx->tile_cnt, ctx->tile_off, ctx->nl_mask, ctx->blk_mask, ctx->tv, ctx->tc, ctx->tp, ctx->v0, ctx->plan_state,
-                 ctx->plans, ctx->hdr, ctx->acc, ctx->cls, ctx->sbout, ctx->arena, ctx->out, ctx->in2, ctx->out2, ctx->tmp, ctx->tmp_used, ctx->big_in, ctx->big_out};
-  for (void *p : dev) if (p) cudaFree(p);
-  void *dev2[] = {ctx->nxt.te, ctx->nxt.se, ctx->nxt.rstart, ctx->nxt.plans, ctx->nxt.hdr};
-  for (void *p : dev2) if (p) cudaFree(p);
-  void *host2[] = {ctx->nxt.h_hdr, ctx->nxt.h_plans, ctx->nxt.h_state};
-  for (void *p : host2) if (p) cudaFreeHost(p);
-  if (ctx->s_prefix) cudaStreamDestroy(ctx->s_prefix);
-  if (ctx->ev_prefix) cudaEventDestroy(ctx->ev_prefix);
-  void *host[] = {ctx->h_hdr, ctx->h_plans, ctx->h_sbout, ctx->h_state, ctx->h_nl, ctx->ring, ctx->hout[0], ctx->hout[1], ctx->hout[2], ctx->hout[3]};
-  for (auto &e : ctx->ev_ring) if (e) cudaEventDestroy(e);
-  for (auto &e : ctx->ev_hout) if (e) cudaEventDestroy(e);
-  for (void *p : host) if (p) cudaFreeHost(p);
-  for (int i = 0; i < 2; ++i) {
-    cudaEvent_t evs[] = {ctx->ev_in[i], ctx->ev_c[i], ctx->ev_out[i], ctx->ev_h0[i], ctx->ev_d0[i]};
-    for (auto e : evs) if (e) cudaEventDestroy(e);
-  }
-  if (ctx->s_in) cudaStreamDestroy(ctx->s_in);
-  if (ctx->s_out) cudaStreamDestroy(ctx->s_out);
-  for (auto &e : ctx->ev) if (e) cudaEventDestroy(e);
-  for (auto &e : ctx->pev) if (e) cudaEventDestroy(e);
-  if (ctx->stream) cudaStreamDestroy(ctx->stream);
-  for (int g = 0; g < GROUPS_MAX; ++g) {
-    if (ctx->gstream[g]) cudaStreamDestroy(ctx->gstream[g]);
-    cudaEvent_t evs[] = {ctx->ev_rb[g], ctx->ev_scan[g], ctx->ev_done[g]};
-    for (auto e : evs) if (e) cudaEventDestroy(e);
-  }
-  if (ctx->hdr_g) cudaFree(ctx->hdr_g);
-  if (ctx->h_hdr_g) cudaFreeHost(ctx->h_hdr_g);
+  cudaSetDevice(ctx->device); /* the handles release their resources on the context's device */
   delete ctx;
 }
 
@@ -175,57 +205,50 @@ static int ctx_init(phy_ctx *ctx, int device, u64 max_batch, u32 max_sb) {
   ctx->out_cap = ctx->max_batch / 2 + (1u << 20);
   ctx->slack = 64 * 1024;
   ctx->max_tiles = (u32)((ctx->max_batch + TILE - 1) / TILE) + 1;
-  int prio_lo = 0, prio_hi = 0; /* the back part's streams outrank the front part's: a front part running ahead only fills gaps */
-  CK(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
-  CK(cudaStreamCreateWithPriority(&ctx->stream, cudaStreamNonBlocking, prio_hi));
-  CK(cudaStreamCreateWithPriority(&ctx->s_prefix, cudaStreamNonBlocking, prio_lo));
-  CK(cudaEventCreateWithFlags(&ctx->ev_prefix, cudaEventDisableTiming));
-  CK(cudaMalloc(&ctx->hdr_g, sizeof(BatchHdr) * GROUPS_MAX));
-  CK(cudaHostAlloc(&ctx->h_hdr_g, sizeof(BatchHdr) * GROUPS_MAX, cudaHostAllocDefault));
-  CK(cudaEventCreateWithFlags(&ctx->ev_rb[0], cudaEventDisableTiming));
-  for (auto &e : ctx->ev) CK(cudaEventCreate(&e));
-  CK(cudaMalloc(&ctx->in, ctx->max_batch + 4096));
-  CK(cudaMemset(ctx->in, 0, ctx->max_batch + 4096));
-  CK(cudaMalloc(&ctx->te, (size_t)(ctx->maxrec + 4) * 4));
-  CK(cudaMalloc(&ctx->se, (size_t)(ctx->maxrec + 4) * 4));
-  CK(cudaMalloc(&ctx->rstart, (size_t)(ctx->maxrec + 4) * 4));
-  CK(cudaMalloc(&ctx->nxt.te, (size_t)(ctx->maxrec + 4) * 4));
-  CK(cudaMalloc(&ctx->nxt.se, (size_t)(ctx->maxrec + 4) * 4));
-  CK(cudaMalloc(&ctx->nxt.rstart, (size_t)(ctx->maxrec + 4) * 4));
-  CK(cudaMalloc(&ctx->kx, (size_t)(ctx->maxrec + 4) * 2));
-  CK(cudaMalloc(&ctx->qoff, (size_t)(ctx->maxrec + 4) * 4));
-  CK(cudaMalloc(&ctx->doff, (size_t)(ctx->maxrec + 4) * 4));
-  CK(cudaMalloc(&ctx->toff, (size_t)(ctx->maxrec + 4) * 4));
+  int prio_lo = 0;
+  CK(cudaDeviceGetStreamPriorityRange(&prio_lo, &ctx->prio_hi));
+  CK(ctx->stream.ensure(ctx->prio_hi));
+  CK(ctx->s_prefix.ensure(prio_lo));
+  CK(ctx->ev_prefix.ensure(cudaEventDisableTiming));
+  CK(ctx->hdr_g.ensure(sizeof(BatchHdr) * GROUPS_MAX));
+  CK(ctx->h_hdr_g.ensure(sizeof(BatchHdr) * GROUPS_MAX));
+  CK(ctx->ev_rb[0].ensure(cudaEventDisableTiming));
+  CK(ctx->ev_k0.ensure(cudaEventDefault));
+  CK(ctx->ev_k1.ensure(cudaEventDefault));
+  CK(ctx->in.ensure(ctx->max_batch + 4096, true));
+  const size_t rec4 = (size_t)(ctx->maxrec + 4) * 4;
+  for (DevBuf<u32> *b : {&ctx->te, &ctx->se, &ctx->rstart, &ctx->nxt.te, &ctx->nxt.se, &ctx->nxt.rstart, &ctx->qoff, &ctx->doff, &ctx->toff})
+    CK(b->ensure(rec4));
+  CK(ctx->kx.ensure((size_t)(ctx->maxrec + 4) * 2));
   {
     size_t rows = (size_t)ctx->maxrec / CH + ctx->max_sb + 2; /* every subblock rounds its chunk count up */
-    CK(cudaMalloc(&ctx->chunk_first, rows * MAXF * 4));
-    CK(cudaMalloc(&ctx->chunk_last, rows * MAXF * 4));
-    CK(cudaMalloc(&ctx->blk_mask, rows * (CH / 32) * 4));
-    CK(cudaMalloc(&ctx->v0, (size_t)ctx->max_sb * MAXF * 4));
+    CK(ctx->chunk_first.ensure(rows * MAXF * 4));
+    CK(ctx->chunk_last.ensure(rows * MAXF * 4));
+    CK(ctx->blk_mask.ensure(rows * (CH / 32) * 4));
+    CK(ctx->v0.ensure((size_t)ctx->max_sb * MAXF * 4));
   }
-  CK(cudaMalloc(&ctx->tile_cnt, (size_t)ctx->max_tiles * 4));
-  CK(cudaMalloc(&ctx->tile_off, (size_t)ctx->max_tiles * 4));
-  CK(cudaMalloc(&ctx->nl_mask, (size_t)ctx->max_tiles * NLT * sizeof(uint2)));
-  CK(cudaMalloc(&ctx->plan_state, sizeof(PlanState)));
-  CK(cudaMalloc(&ctx->plans, sizeof(SbPlan) * ctx->max_sb));
-  CK(cudaMalloc(&ctx->hdr, sizeof(BatchHdr)));
-  CK(cudaMalloc(&ctx->nxt.plans, sizeof(SbPlan) * ctx->max_sb));
-  CK(cudaMalloc(&ctx->nxt.hdr, sizeof(BatchHdr)));
-  CK(cudaMalloc(&ctx->acc, sizeof(SbAcc) * ctx->max_sb));
-  CK(cudaMalloc(&ctx->cls, sizeof(SbClass) * ctx->max_sb));
-  CK(cudaMalloc(&ctx->sbout, sizeof(SbOut) * ctx->max_sb));
-  CK(cudaMalloc(&ctx->arena, (size_t)ctx->arena_words * 4 * ctx->max_sb));
-  CK(cudaMalloc(&ctx->out, ctx->out_cap + 64));
-  ctx->tmp_cap = (ctx->max_batch + ctx->max_batch / 2) / 4 + (1u << 20); /* 1.5 bytes per input byte: slots are sized by bounds, not by what is written */
-  CK(cudaMalloc(&ctx->tmp, ctx->tmp_cap * 4));
-  CK(cudaMalloc(&ctx->tmp_used, sizeof(u64)));
-  CK(cudaHostAlloc(&ctx->h_hdr, sizeof(BatchHdr), cudaHostAllocDefault));
-  CK(cudaHostAlloc(&ctx->h_plans, sizeof(SbPlan) * ctx->max_sb, cudaHostAllocDefault));
-  CK(cudaHostAlloc(&ctx->h_sbout, sizeof(SbOut) * ctx->max_sb, cudaHostAllocDefault));
-  CK(cudaHostAlloc(&ctx->h_state, sizeof(PlanState), cudaHostAllocDefault));
-  CK(cudaHostAlloc(&ctx->nxt.h_hdr, sizeof(BatchHdr), cudaHostAllocDefault));
-  CK(cudaHostAlloc(&ctx->nxt.h_plans, sizeof(SbPlan) * ctx->max_sb, cudaHostAllocDefault));
-  CK(cudaHostAlloc(&ctx->nxt.h_state, sizeof(PlanState), cudaHostAllocDefault));
+  CK(ctx->tile_cnt.ensure((size_t)ctx->max_tiles * 4));
+  CK(ctx->tile_off.ensure((size_t)ctx->max_tiles * 4));
+  CK(ctx->nl_mask.ensure((size_t)ctx->max_tiles * NLT * sizeof(uint2)));
+  CK(ctx->plan_state.ensure(sizeof(PlanState)));
+  CK(ctx->plans.ensure(sizeof(SbPlan) * ctx->max_sb));
+  CK(ctx->hdr.ensure(sizeof(BatchHdr)));
+  CK(ctx->nxt.plans.ensure(sizeof(SbPlan) * ctx->max_sb));
+  CK(ctx->nxt.hdr.ensure(sizeof(BatchHdr)));
+  CK(ctx->acc.ensure(sizeof(SbAcc) * ctx->max_sb));
+  CK(ctx->cls.ensure(sizeof(SbClass) * ctx->max_sb));
+  CK(ctx->sbout.ensure(sizeof(SbOut) * ctx->max_sb));
+  CK(ctx->arena.ensure((size_t)ctx->arena_words * 4 * ctx->max_sb));
+  CK(ctx->out.ensure(ctx->out_cap + 64));
+  CK(ctx->tmp.ensure(((ctx->max_batch + ctx->max_batch / 2) / 4 + (1u << 20)) * 4)); /* 1.5 bytes per input byte: slots are sized by bounds, not by what is written */
+  CK(ctx->tmp_used.ensure(sizeof(u64)));
+  CK(ctx->h_hdr.ensure(sizeof(BatchHdr)));
+  CK(ctx->h_plans.ensure(sizeof(SbPlan) * ctx->max_sb));
+  CK(ctx->h_sbout.ensure(sizeof(SbOut) * ctx->max_sb));
+  CK(ctx->h_state.ensure(sizeof(PlanState)));
+  CK(ctx->nxt.h_hdr.ensure(sizeof(BatchHdr)));
+  CK(ctx->nxt.h_plans.ensure(sizeof(SbPlan) * ctx->max_sb));
+  CK(ctx->nxt.h_state.ensure(sizeof(PlanState)));
   {
     u8 lut[256];
     fill_char_lut(lut);
@@ -278,11 +301,21 @@ extern "C" int64_t phy_find_first_record(const uint8_t *b, uint64_t lim) {
   return (int64_t)((b[c + 1] == '@') ? c + 1 : first_at);
 }
 
-static const bool dbg_sync = getenv("PHY_DEBUG_SYNC") != nullptr; /* fault isolation: synchronise after every launch */
+/* Switches of the environment, read once per process:
+ *   PHY_GROUPS      subblock groups of a batch (1..GROUPS_MAX, default 3; the profiling scripts set 1)
+ *   PHY_ENC=0       every subblock through the two-walk encoder (k_lengths + k_emit) instead of the single-walk kernels
+ *   PHY_DEBUG_SYNC  fault isolation: synchronise after every launch (also runs one group and no front part ahead) */
+static int env_int(const char *name, int dflt) { const char *v = getenv(name); return v ? atoi(v) : dflt; }
+static const struct {
+  int groups = env_int("PHY_GROUPS", 3); /* measured on 1 GB: 3.25 / 3.13 / 3.01 / 3.05 ms for 1..4 groups */
+  bool enc = env_int("PHY_ENC", 1) != 0;
+  bool debug_sync = getenv("PHY_DEBUG_SYNC") != nullptr;
+} sw;
+
 #define PMARK()                                                                                                   \
   do {                                                                                                            \
     if (ctx->profile) cudaEventRecord(ctx->pev[ctx->pi], st);                                                     \
-    if (dbg_sync) {                                                                                               \
+    if (sw.debug_sync) {                                                                                          \
       cudaError_t e_ = cudaStreamSynchronize(st);                                                                 \
       if (e_ == cudaSuccess) e_ = cudaGetLastError();                                                             \
       if (e_ != cudaSuccess) {                                                                                    \
@@ -293,18 +326,61 @@ static const bool dbg_sync = getenv("PHY_DEBUG_SYNC") != nullptr; /* fault isola
     ++ctx->pi;                                                                                                    \
   } while (0)
 
-/* Front part of a batch on stream `st`: record splitter, window chain, sizes; its results go to the "next" set and are copied
- * to that set's host mirrors.  Does not wait.  `start_pos` = first record of the next window inside the batch. */
-static int prefix_launch(phy_ctx *ctx, cudaStream_t st, const u8 *in, u32 len, u32 start_pos, i64 batch_base, i64 region_len, bool is_final) {
+/* Where the batch walk over a region stands; every entry point walks a region by these rules.  A batch is the region's
+ * bytes [base, base + blen); its window chain starts at next_pos. */
+struct Walk {
+  PlanState st;           /* the reference's plan state at the region's start (walk_init) */
+  u64 len = 0;            /* region bytes */
+  u64 max_batch = 0;
+  u64 back = 0;           /* how far before a batch's end the next one starts: a window that does not fit the rest of a batch
+                           * (with the slack for records longer than the overlap) is left to the next batch */
+  u64 base = 0, blen = 0;
+  bool final = false;     /* the batch ends at the region's end */
+  bool nl = false;        /* last rank whose file does not end in a newline: the reference's arithmetic still places the next
+                           * record start one byte past the end; a virtual newline behind the final batch gives the splitter
+                           * the same view (written by a one-byte memset behind the region's bytes on the device) */
+  u64 next_pos = 0;       /* PlanState::bytes_read at the start of the batch */
+  u32 nb = 0;             /* batches finished */
+
+  u64 len_at(u64 b) const { return len - b < max_batch ? len - b : max_batch; }
+  void place(u64 b) { base = b; blen = len_at(b); final = b + blen == len; }
+  /* start of the batch after a non-final one */
+  u64 candidate() const { return (base + blen - back) & ~(u64)255; }
+  u32 kernel_len() const { return (u32)(blen + (final && nl ? 1 : 0)); }
+  u32 start_pos() const { return (u32)(next_pos - base) + (nb == 0 ? st.rec_start : 0u); }
+  /* After a batch whose front part made S windows and left the chain at hs: `done` once the working region is covered,
+   * else `move` says whether the next round runs the candidate batch or -- the chain stopped early because the batch's
+   * subblock capacity was used up -- the same bytes again.  A chain that made no progress is an error. */
+  int after(phy_ctx *ctx, const PlanState &hs, u32 S, bool &done, bool &move) {
+    ++nb;
+    move = false;
+    if (hs.status) { ctx->err = std::string("window chaining failed: ") + phy_strerror(hs.status); return hs.status; }
+    done = hs.done != 0;
+    if (done) return PHY_OK;
+    const u64 stopped = (u64)hs.bytes_read;
+    if (S == 0 && stopped == next_pos && (final || stopped < candidate())) {
+      ctx->err = final ? "region exhausted before the working region was covered" : "a window does not fit one batch (raise max_batch_bytes)";
+      return final ? PHY_ERR_MALFORMED : PHY_ERR_CAPACITY;
+    }
+    next_pos = stopped;
+    move = !final && next_pos >= candidate();
+    return PHY_OK;
+  }
+};
+
+/* Front part of the walk's batch on stream `st` (`in`: the batch's first byte on the device): record splitter, window chain,
+ * sizes; its results go to the "next" set and are copied to that set's host mirrors.  Does not wait. */
+static int prefix_launch(phy_ctx *ctx, cudaStream_t st, const u8 *in, const Walk &w) {
+  const u32 len = w.kernel_len();
   Dev d;
   memset(&d, 0, sizeof d);
-  d.in = in; d.len = len; d.start_pos = start_pos;
+  d.in = in; d.len = len; d.start_pos = w.start_pos();
   d.te = ctx->nxt.te; d.se = ctx->nxt.se; d.rstart = ctx->nxt.rstart; d.maxrec = ctx->maxrec;
   d.tile_cnt = ctx->tile_cnt; d.tile_off = ctx->tile_off; d.nl_mask = ctx->nl_mask; d.ntiles = (len + TILE - 1) / TILE;
   d.plan_state = ctx->plan_state; d.plans = ctx->nxt.plans; d.max_sb = ctx->max_sb; d.hdr = ctx->nxt.hdr;
-  d.batch_base = batch_base; d.region_len = region_len; d.batch_is_final = is_final ? 1 : 0; d.slack = ctx->slack;
-  ctx->nxt_args.in = in; ctx->nxt_args.len = len; ctx->nxt_args.start_pos = start_pos; ctx->nxt_args.batch_base = batch_base;
-  ctx->nxt_args.region_len = region_len; ctx->nxt_args.is_final = is_final;
+  d.batch_base = (i64)w.base; d.region_len = (i64)w.len; d.batch_is_final = w.final ? 1 : 0; d.slack = ctx->slack;
+  ctx->nxt_args.in = in; ctx->nxt_args.len = len; ctx->nxt_args.start_pos = d.start_pos; ctx->nxt_args.batch_base = d.batch_base;
+  ctx->nxt_args.region_len = d.region_len; ctx->nxt_args.is_final = w.final;
   if (d.ntiles == 0) { ctx->err = "empty batch"; return PHY_ERR_ARG; }
   ctx->pi = 0;
   PMARK();
@@ -325,9 +401,9 @@ static int prefix_launch(phy_ctx *ctx, cudaStream_t st, const u8 *in, u32 len, u
 /* Waits for the front part launched last and makes its results the current set: h_hdr / h_state / h_plans describe the batch. */
 static int prefix_finish(phy_ctx *ctx) {
   CK(cudaEventSynchronize(ctx->ev_prefix));
-  std::swap(ctx->te, ctx->nxt.te); std::swap(ctx->se, ctx->nxt.se); std::swap(ctx->rstart, ctx->nxt.rstart);
-  std::swap(ctx->plans, ctx->nxt.plans); std::swap(ctx->hdr, ctx->nxt.hdr);
-  std::swap(ctx->h_hdr, ctx->nxt.h_hdr); std::swap(ctx->h_plans, ctx->nxt.h_plans); std::swap(ctx->h_state, ctx->nxt.h_state);
+  ctx->te.swap(ctx->nxt.te); ctx->se.swap(ctx->nxt.se); ctx->rstart.swap(ctx->nxt.rstart);
+  ctx->plans.swap(ctx->nxt.plans); ctx->hdr.swap(ctx->nxt.hdr);
+  ctx->h_hdr.swap(ctx->nxt.h_hdr); ctx->h_plans.swap(ctx->nxt.h_plans); ctx->h_state.swap(ctx->nxt.h_state);
   ctx->cur_args = ctx->nxt_args;
   ctx->last_S = 0;
   const BatchHdr &H = *ctx->h_hdr;
@@ -352,7 +428,7 @@ static int run_body(phy_ctx *ctx, u8 *out, u64 out_cap) {
   d.out = out; d.out_cap = out_cap;
   d.batch_base = A.batch_base; d.region_len = A.region_len; d.batch_is_final = A.is_final ? 1 : 0; d.slack = ctx->slack;
   d.span_bytes = 0;
-  d.tmp = ctx->tmp; d.tmp_cap = ctx->tmp_cap; d.tmp_used = ctx->tmp_used;
+  d.tmp = ctx->tmp; d.tmp_cap = ctx->tmp.cap / 4; d.tmp_used = ctx->tmp_used;
   cudaStream_t st = ctx->stream;
   if (ctx->prev_groups) { /* the previous batch is complete (the callers synchronise): its alphabet is the hint for this one */
     u32 mx = 0, mq = 0;
@@ -374,15 +450,8 @@ static int run_body(phy_ctx *ctx, u8 *out, u64 out_cap) {
     const u64 chunks = (u64)PL.chunk_base + (PL.n_records + CH - 1) / CH;
     d.nfs = d.max_nf ? d.max_nf : 1u;
     const u64 need = chunks * d.nfs * CH;
-    if (need > ctx->tv_cap) {
-      if (ctx->tv) { CK(cudaFree(ctx->tv)); ctx->tv = nullptr; }
-      if (ctx->tp) { CK(cudaFree(ctx->tp)); ctx->tp = nullptr; }
-      if (ctx->tc) { CK(cudaFree(ctx->tc)); ctx->tc = nullptr; }
-      ctx->tv_cap = 0;
-      const u64 cap = need + need / 4;
-      CK(cudaMalloc(&ctx->tv, cap * 4)); CK(cudaMalloc(&ctx->tp, cap * 4)); CK(cudaMalloc(&ctx->tc, cap * 4));
-      ctx->tv_cap = cap;
-    }
+    for (DevBuf<u32> *b : {&ctx->tv, &ctx->tp, &ctx->tc})
+      if (b->cap < need * 4) CK(b->ensure((need + need / 4) * 4));
     d.tv = ctx->tv; d.tp = ctx->tp; d.tc = ctx->tc;
   }
   /* launch geometry shared by all subblock groups of the batch */
@@ -393,28 +462,22 @@ static int run_body(phy_ctx *ctx, u8 *out, u64 out_cap) {
   /* Single-walk encoder (phy_encode.cuh): G lanes share a record's quality / DNA codes so that a lane's run of read
    * positions stays short (its staging words and the records a warp keeps staged shrink with G); PHY_ENC=0 switches
    * the single-walk kernels off (every subblock then takes k_lengths + k_emit). */
-  static const int enc_env = getenv("PHY_ENC") ? atoi(getenv("PHY_ENC")) : 1;
-  static const int encg_env = getenv("PHY_ENC_G") ? atoi(getenv("PHY_ENC_G")) : 0;
-  static const int qdbuf_env = getenv("PHY_QD_NBUF") ? atoi(getenv("PHY_QD_NBUF")) : 0;
   u32 encG = H.max_len <= 64 ? 1u : H.max_len <= 256 ? 4u : 8u; /* measured per shape (36 / 100 / 150 / 50-205 bp): 1, 4, 4, 4 */
-  if (encg_env == 1 || encg_env == 2 || encg_env == 4 || encg_env == 8) encG = (u32)encg_env;
   while (encG < 8 && seg_len(H.max_len, encG) > 64) encG *= 2; /* a lane keeps one bit per position of its run (k_seqstat) */
-  d.fg.g = enc_env ? encG : 0u;
+  d.fg.g = sw.enc ? encG : 0u;
   /* lane-private staging: a lane's run of positions times the longest quality code -- 12 bits unless the previous batch
    * of this context saw longer ones (subblocks that need more than the kernels were launched with take the two-walk path) */
   d.fg.lpw_q = (seg_len(H.max_len, encG) * (ctx->qcode_hint > 12 ? (ctx->qcode_hint > 24 ? 24u : ctx->qcode_hint) : 12u) + 31u) / 32u + 2u;
   d.fg.pk_bytes = 0;
   d.qd_stage = ((32u / encG) * H.max_rec + 32u + 255u) & ~255u;
   if (encG == 1) d.qd_stage = (H.max_span32 + 16 + 255) & ~255u;
-  d.qd_nbuf = qdbuf_env == 1 || qdbuf_env == 2 ? (u32)qdbuf_env : (encG > 1 && d.qd_stage <= 2560 ? 2u : 1u); /* measured: a second stage only pays while it is small (100 bp: 0.86 vs 0.90 ms per GB, 150 bp: 0.89 vs 0.78) */
+  d.qd_nbuf = encG > 1 && d.qd_stage <= 2560 ? 2u : 1u; /* measured: a second stage only pays while it is small (100 bp: 0.86 vs 0.90 ms per GB, 150 bp: 0.89 vs 0.78) */
   d.ts = (((H.max_tlen + 16u + 15u) & ~15u) | 16u);
   const u32 max_tasks = (H.max_chunks * CH + TASK_RECORDS - 1) / TASK_RECORDS;
   /* statistics: k_seqstat uses the lane split and the record stages of k_enc_qd, k_stat1 / k_stat2 stage title lines only */
   d.sq_rows = H.max_len < 1 ? 1u : H.max_len > RAW_ROWS - 1 ? RAW_ROWS - 1 : H.max_len;
-  static const int sqbuf_env = getenv("PHY_SQ_NBUF") ? atoi(getenv("PHY_SQ_NBUF")) : 0;
-  d.sq_stage = d.qd_stage; d.sq_nbuf = sqbuf_env == 2 ? 2u : 1u; /* one stage: more resident CTAs hide the copy better (100 bp: 0.66 vs 0.76 ms per GB) */
-  static const int sqwide_env = getenv("PHY_SQ_WIDE") ? atoi(getenv("PHY_SQ_WIDE")) : 126;
-  const bool sq_wide = d.sq_rows <= (u32)sqwide_env; /* 32-bit counters while the private table stays below 48 KB, else 16-bit pairs */
+  d.sq_stage = d.qd_stage; d.sq_nbuf = 1; /* one stage: more resident CTAs hide the copy better (100 bp: 0.66 vs 0.76 ms per GB) */
+  const bool sq_wide = d.sq_rows <= 126; /* 32-bit counters while the private table stays below 48 KB, else 16-bit pairs */
   const u32 sq_dyn = ((d.sq_rows * (sq_wide ? 97u : SQ_ROWW) * 4u + 15u) & ~15u) + SQ_WARPS * d.sq_nbuf * d.sq_stage;
   /* k_stat1: two stages of one title slot per lane for every warp; fewer warps per CTA when the title lines are long */
   u32 s1_warps = S1W;
@@ -426,17 +489,12 @@ static int run_body(phy_ctx *ctx, u8 *out, u64 out_cap) {
    * in k_huff, one CTA per subblock in k_layout): while one group sits in such a stage the other keeps the SMs busy.
    * A group sees its own slice of the per-subblock arrays (shifted base pointers) and its own header; the payloads of all
    * groups still lie back to back because a group's output scan starts at the previous group's end. */
-  static const int groups_env = getenv("PHY_GROUPS") ? atoi(getenv("PHY_GROUPS")) : 3; /* measured on 1 GB: 3.25 / 3.13 / 3.01 / 3.05 ms for 1..4 groups */
-  u32 G = (ctx->profile || dbg_sync || S < 16) ? 1u : (u32)(groups_env < 1 ? 1 : groups_env > GROUPS_MAX ? GROUPS_MAX : groups_env);
-  if (G > 1 && !ctx->gstream[1]) {
-    int prio_lo = 0, prio_hi = 0;
-    CK(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
-    for (int g = 1; g < GROUPS_MAX; ++g) CK(cudaStreamCreateWithPriority(&ctx->gstream[g], cudaStreamNonBlocking, prio_hi));
-    for (int g = 0; g < GROUPS_MAX; ++g) {
-      if (g) CK(cudaEventCreateWithFlags(&ctx->ev_rb[g], cudaEventDisableTiming));
-      CK(cudaEventCreateWithFlags(&ctx->ev_scan[g], cudaEventDisableTiming)); CK(cudaEventCreateWithFlags(&ctx->ev_done[g], cudaEventDisableTiming));
+  const u32 G = (ctx->profile || sw.debug_sync || S < 16) ? 1u : (u32)(sw.groups < 1 ? 1 : sw.groups > GROUPS_MAX ? GROUPS_MAX : sw.groups);
+  if (G > 1)
+    for (u32 g = 0; g < G; ++g) {
+      if (g) CK(ctx->gstream[g].ensure(ctx->prio_hi));
+      for (Event *e : {&ctx->ev_rb[g], &ctx->ev_scan[g], &ctx->ev_done[g]}) CK(e->ensure(cudaEventDisableTiming));
     }
-  }
   Dev dg[GROUPS_MAX];
   u32 s0[GROUPS_MAX + 1];
   for (u32 g = 0; g <= G; ++g) s0[g] = (u32)((u64)S * g / G);
@@ -486,9 +544,7 @@ static int run_body(phy_ctx *ctx, u8 *out, u64 out_cap) {
     k_dnacount<<<dim3((H.max_chunks + S2G - 1) / S2G, Sg), CH, span, gs>>>(e); /* returns at once unless the DNA is Huffman coded */
     GMARK();
   }
-  static const int pair_env = getenv("PHY_EMIT_PAIR") ? atoi(getenv("PHY_EMIT_PAIR")) : -1;
-  static const bool pk_exact = getenv("PHY_PK_EXACT") != nullptr;
-  const u32 nq_hint = pk_exact ? 0u : ctx->nq_hint; /* quality alphabet of the previous batch of this context (0: none yet) */
+  const u32 nq_hint = ctx->nq_hint; /* quality alphabet of the previous batch of this context (0: none yet) */
   for (u32 g = 0; g < G; ++g) {
     Dev &e = dg[g];
     const u32 Sg = s0[g + 1] - s0[g];
@@ -522,7 +578,7 @@ static int run_body(phy_ctx *ctx, u8 *out, u64 out_cap) {
     /* two-walk kernels for the subblocks the single-walk kernels could not take (bounds beyond their staging): one warp
      * per 32-record block while at least ~32 warps of such CTAs fit an SM, else warp pairs on a shared stage */
     const u32 solo_dyn = e.pk_bytes + EW * e.enc_stage, pair_dyn = e.pk_bytes + EP * e.enc_stage;
-    const bool pair = pair_env >= 0 ? pair_env != 0 : (solo_dyn + 7 * 1024) * 4 > 227u * 1024;
+    const bool pair = (solo_dyn + 7 * 1024) * 4 > 227u * 1024;
     const dim3 ge_solo((4 * H.max_chunks + EW * EGW - 1) / (EW * EGW), Sg), ge_pair((4 * H.max_chunks + EP * EGW - 1) / (EP * EGW), Sg);
     if (pair) k_lengths<true><<<ge_pair, EW * 32, pair_dyn, gs>>>(e);
     else k_lengths<false><<<ge_solo, EW * 32, solo_dyn, gs>>>(e);
@@ -553,9 +609,9 @@ static int run_body(phy_ctx *ctx, u8 *out, u64 out_cap) {
   return PHY_OK;
 }
 
-/* Front and back part of one batch one after the other on the main stream (the pipelined region call; profiling). */
-static int run_batch(phy_ctx *ctx, const u8 *in, u8 *out, u64 out_cap, u32 len, u32 start_pos, i64 batch_base, i64 region_len, bool is_final) {
-  int rc = prefix_launch(ctx, ctx->stream, in, len, start_pos, batch_base, region_len, is_final);
+/* Front and back part of the walk's batch one after the other on the main stream (the pipelined region call). */
+static int run_batch(phy_ctx *ctx, const u8 *in, u8 *out, u64 out_cap, const Walk &w) {
+  int rc = prefix_launch(ctx, ctx->stream, in, w);
   if (rc) return rc;
   rc = prefix_finish(ctx);
   if (rc) return rc;
@@ -574,36 +630,61 @@ static void fill_descs(phy_ctx *ctx, u32 S, u64 out_base, phy_subblock_desc *des
   }
 }
 
-static int init_plan(phy_ctx *ctx, const uint8_t *region_host, u64 region_len, const phy_region_params *p, u32 first_rec_start_known,
-                     bool have_first, PlanState &st) {
+static const u64 HEAD_BYTES = 1u << 20; /* the '@' heuristic of a rank > 0 looks at this much of the region's head */
+
+/* Region set-up of every walk: the parameters, the first record of a rank > 0 (found in `head`, the region's first
+ * min(region_len, HEAD_BYTES) bytes on the host), the reference's plan state (uploaded on the main stream) and the first
+ * batch.  The caller decides Walk::nl. */
+static int walk_init(phy_ctx *ctx, const u8 *head, u64 region_len, const phy_region_params *p, Walk &w) {
   if (!p || p->np < 1 || p->rank < 0 || p->rank >= p->np || p->window_bytes == 0 || p->file_size == 0) { ctx->err = "bad region parameters"; return PHY_ERR_ARG; }
   u32 first = 0;
   if (p->rank != 0) {
-    if (have_first) first = first_rec_start_known;
-    else {
-      int64_t f = phy_find_first_record(region_host, region_len < (1u << 20) ? region_len : (1u << 20)); /* the caller has waited for this much */
-      if (f < 0) { ctx->err = "no record start found at the beginning of the region"; return (int)f; }
-      first = (u32)f;
-    }
+    int64_t f = phy_find_first_record(head, region_len < HEAD_BYTES ? region_len : HEAD_BYTES);
+    if (f < 0) { ctx->err = "no record start found at the beginning of the region"; return (int)f; }
+    first = (u32)f;
   }
-  plan_init(st, p->file_size, p->np, p->rank, p->window_bytes, p->overlap, p->record_cap, first, p->threads);
-  if ((u64)st.wr_len > region_len) { ctx->err = "region_len is shorter than the rank's working region"; return PHY_ERR_ARG; }
+  plan_init(w.st, p->file_size, p->np, p->rank, p->window_bytes, p->overlap, p->record_cap, first, p->threads);
+  if ((u64)w.st.wr_len > region_len) { ctx->err = "region_len is shorter than the rank's working region"; return PHY_ERR_ARG; }
+  w.len = region_len; w.max_batch = ctx->max_batch; w.back = (u64)p->window_bytes + ctx->slack;
+  if (region_len > ctx->max_batch && ctx->max_batch < 2 * w.back + 4096) { ctx->err = "max_batch_bytes is too small for the window size"; return PHY_ERR_CAPACITY; }
+  w.place(0);
+  *ctx->h_state = w.st;
+  ctx->launches = 0;
+  CK(cudaMemcpyAsync(ctx->plan_state, ctx->h_state, sizeof(PlanState), cudaMemcpyHostToDevice, ctx->stream));
   return PHY_OK;
+}
+
+/* Totals of a walk's descriptors. */
+struct Tally {
+  u32 n = 0;
+  u64 bytes_in = 0, bytes_out = 0;
+  int worst = 0;
+  void add(const phy_subblock_desc *d, u32 k) {
+    for (u32 i = 0; i < k; ++i) { bytes_in += d[i].bytes_consumed; bytes_out += d[i].out_len; if (d[i].status < worst) worst = d[i].status; }
+    n += k;
+  }
+};
+
+/* Fills *r (if given) and returns the worst subblock status. */
+static int walk_result(phy_ctx *ctx, const Walk &w, const Tally &t, u64 out_used, float kernel_ms, float h2d_ms, float d2h_ms, phy_region_result *r) {
+  if (r) {
+    memset(r, 0, sizeof *r);
+    r->n_subblocks = t.n; r->n_batches = w.nb; r->wr_overlap = (int32_t)w.st.rec_start; r->kernel_launches = ctx->launches;
+    r->out_used = out_used; r->kernel_ms = kernel_ms; r->h2d_ms = h2d_ms; r->d2h_ms = d2h_ms;
+    r->bytes_in = t.bytes_in; r->bytes_out = t.bytes_out;
+  }
+  if (t.worst) ctx->err = std::string("a subblock failed: ") + phy_strerror(t.worst);
+  return t.worst;
 }
 
 extern "C" int phy_upload(phy_ctx *ctx, const uint8_t *region, uint64_t region_len) {
   if (!ctx || !region || region_len == 0) return PHY_ERR_ARG;
   CK(cudaSetDevice(ctx->device));
+  ctx->resident_len = ctx->resident_out = 0; /* until the new bytes are in place */
   u8 *dst = ctx->in;
   if (region_len > ctx->max_batch) { /* larger than one batch: its own device buffers, walked batch by batch */
-    if (ctx->big_in_cap < region_len) {
-      if (ctx->big_in) { CK(cudaFree(ctx->big_in)); ctx->big_in = nullptr; }
-      if (ctx->big_out) { CK(cudaFree(ctx->big_out)); ctx->big_out = nullptr; }
-      CK(cudaMalloc(&ctx->big_in, region_len + 4096));
-      ctx->big_in_cap = region_len;
-      ctx->big_out_cap = region_len / 2 + (1u << 20);
-      CK(cudaMalloc(&ctx->big_out, ctx->big_out_cap + 64));
-    }
+    CK(ctx->big_in.ensure(region_len + 4096));
+    CK(ctx->big_out.ensure(region_len / 2 + (1u << 20) + 64));
     dst = ctx->big_in;
   }
   for (u64 o = 0; o < region_len; o += 1ull << 30) { /* 1 GiB pieces: pageable sources are staged by the driver */
@@ -617,10 +698,6 @@ extern "C" int phy_upload(phy_ctx *ctx, const uint8_t *region, uint64_t region_l
   return PHY_OK;
 }
 
-/* How far before a batch's end the next one starts: a window that does not fit the rest of a batch (with the slack for
- * records longer than the overlap) is left to the next batch, which therefore starts one window + slack earlier. */
-static u64 batch_back(const phy_ctx *ctx, const phy_region_params *p) { return (u64)p->window_bytes + ctx->slack; }
-
 extern "C" int phy_compress_resident(phy_ctx *ctx, uint64_t region_len, const phy_region_params *params,
                                      phy_subblock_desc *descs, uint32_t *inout_n_descs, phy_region_result *result) {
   if (!ctx || !descs || !inout_n_descs) return PHY_ERR_ARG;
@@ -628,97 +705,60 @@ extern "C" int phy_compress_resident(phy_ctx *ctx, uint64_t region_len, const ph
   CK(cudaSetDevice(ctx->device));
   const bool big = region_len > ctx->max_batch;
   u8 *rin = big ? ctx->big_in : ctx->in, *rout = big ? ctx->big_out : ctx->out;
-  const u64 rout_cap = big ? ctx->big_out_cap : ctx->out_cap;
-  PlanState st;
-  u32 first = 0;
-  if (params && params->rank != 0) {
-    /* the head of the region is needed on the host for the '@' heuristic */
-    u64 n = region_len < 65536 ? region_len : 65536;
-    std::string head(n, '\0');
-    CK(cudaMemcpy(&head[0], rin, n, cudaMemcpyDeviceToHost));
-    int64_t f = phy_find_first_record((const uint8_t *)head.data(), n);
-    if (f < 0) { ctx->err = "no record start found at the beginning of the region"; return (int)f; }
-    first = (u32)f;
+  const u64 rout_cap = big ? ctx->big_out.cap - 64 : ctx->out_cap;
+  cudaStream_t s = ctx->stream;
+  std::vector<u8> head;
+  if (params && params->rank != 0) { /* the head of the region is needed on the host for the '@' heuristic */
+    head.resize(region_len < HEAD_BYTES ? region_len : HEAD_BYTES);
+    CK(cudaMemcpy(head.data(), rin, head.size(), cudaMemcpyDeviceToHost));
   }
-  int rc = init_plan(ctx, nullptr, region_len, params, first, true, st);
+  Walk w;
+  int rc = walk_init(ctx, head.data(), region_len, params, w);
   if (rc) return rc;
-  u64 len_total = region_len;
-  if (st.is_last) { /* last rank whose file does not end in a newline: a virtual one (see patch_trailing_newline) */
+  if (w.st.is_last) {
     u8 last_byte = '\n';
     CK(cudaMemcpy(&last_byte, rin + region_len - 1, 1, cudaMemcpyDeviceToHost));
-    if (last_byte != '\n') { const u8 nl = '\n'; CK(cudaMemcpy(rin + region_len, &nl, 1, cudaMemcpyHostToDevice)); len_total += 1; }
+    w.nl = last_byte != '\n';
+    if (w.nl) CK(cudaMemsetAsync(rin + region_len, '\n', 1, s));
   }
-  const u64 back = batch_back(ctx, params);
-  if (big && ctx->max_batch < 2 * back + 4096) { ctx->err = "max_batch_bytes is too small for the window size"; return PHY_ERR_CAPACITY; }
-  *ctx->h_state = st;
-  ctx->launches = 0;
-  cudaStream_t s = ctx->stream;
-  CK(cudaMemcpyAsync(ctx->plan_state, ctx->h_state, sizeof(PlanState), cudaMemcpyHostToDevice, s));
-  CK(cudaEventRecord(ctx->ev[0], s));
+  CK(cudaEventRecord(ctx->ev_k0, s));
   /* The front part of batch b + 1 (record splitter, window chain: bandwidth- and latency-bound, 0.5 ms per GB) runs on a
    * lower-priority stream beside the back part of batch b (issue-bound record kernels); it only needs to know where batch
-   * b's chain stopped, which batch b's own front part has already told the host. */
-  static const bool pipe_env = !(getenv("PHY_PIPE") && atoi(getenv("PHY_PIPE")) == 0);
-  const bool pipelined = pipe_env && !ctx->profile && !dbg_sync;
-  cudaStream_t sp = pipelined ? ctx->s_prefix : s;
-  if (pipelined) { CK(cudaEventRecord(ctx->ev[2], s)); CK(cudaStreamWaitEvent(sp, ctx->ev[2], 0)); } /* the plan state is on the device first */
+   * b's chain stopped, which batch b's own front part has already told the host.  Profiling and PHY_DEBUG_SYNC run each
+   * batch's front part on the main stream after the back part of the batch before. */
+  const bool ahead = !ctx->profile && !sw.debug_sync;
+  cudaStream_t sp = ahead ? ctx->s_prefix : s;
+  if (ahead) CK(cudaStreamWaitEvent(sp, ctx->ev_k0, 0)); /* the plan state is on the device first */
   const u32 cap_descs = *inout_n_descs;
-  u32 nd = 0, nb = 0;
-  u64 base = 0, next_pos = 0, out_used = 0;
-  bool done = false;
-  u64 blen = len_total < ctx->max_batch ? len_total : ctx->max_batch;
-  bool final = blen == len_total;
-  rc = prefix_launch(ctx, sp, rin, (u32)blen, first, 0, (i64)len_total, final);
+  Tally t;
+  u64 out_used = 0;
+  rc = prefix_launch(ctx, sp, rin, w);
   if (rc) return rc;
-  while (!done) {
+  for (bool done = false; !done;) {
     rc = prefix_finish(ctx);
     if (rc) return rc;
     const u32 S = ctx->last_S;
-    const PlanState hs = *ctx->h_state;
-    if (hs.status) { ctx->err = std::string("window chaining failed: ") + phy_strerror(hs.status); return hs.status; }
-    if (nd + S > cap_descs) { ctx->err = "descriptor array too small"; return PHY_ERR_CAPACITY; }
-    done = hs.done != 0;
-    u64 nbase = base, nblen = 0;
-    bool nfinal = false;
-    if (!done) {
-      if (S == 0 && (u64)hs.bytes_read == next_pos && (final || (u64)hs.bytes_read < base + blen - back)) {
-        ctx->err = final ? "region exhausted before the working region was covered" : "a window does not fit one batch (raise max_batch_bytes)";
-        return final ? PHY_ERR_MALFORMED : PHY_ERR_CAPACITY;
-      }
-      next_pos = (u64)hs.bytes_read;
-      /* the chain stops early when the batch's subblock capacity is used up: the next round starts where it stopped,
-       * in the same bytes; otherwise the next batch starts one window + slack before this one's end */
-      const u64 cand = final ? base : (base + blen - back) & ~(u64)255;
-      if (next_pos >= cand) nbase = cand;
-      nblen = len_total - nbase;
-      if (nblen > ctx->max_batch) nblen = ctx->max_batch;
-      nfinal = nbase + nblen == len_total;
-    }
+    bool move;
+    rc = w.after(ctx, *ctx->h_state, S, done, move);
+    if (rc) return rc;
+    if (t.n + S > cap_descs) { ctx->err = "descriptor array too small"; return PHY_ERR_CAPACITY; }
+    if (move) w.place(w.candidate());
     rc = run_body(ctx, rout + out_used, rout_cap - out_used); /* first, so that the GPU is busy again as early as possible ... */
     if (rc) return rc;
-    if (!done && pipelined) { rc = prefix_launch(ctx, sp, rin + nbase, (u32)nblen, (u32)(next_pos - nbase), (i64)nbase, (i64)len_total, nfinal); if (rc) return rc; } /* ... the next front part fills in beside it */
+    if (!done && ahead) { rc = prefix_launch(ctx, sp, rin + w.base, w); if (rc) return rc; } /* ... the next front part fills in beside it */
     CK(cudaStreamSynchronize(s));
-    fill_descs(ctx, S, out_used, descs + nd);
-    nd += S; ++nb;
+    fill_descs(ctx, S, out_used, descs + t.n);
+    t.add(descs + t.n, S);
     if (S) out_used += ctx->h_hdr->total_out;
-    if (!done && !pipelined) { rc = prefix_launch(ctx, sp, rin + nbase, (u32)nblen, (u32)(next_pos - nbase), (i64)nbase, (i64)len_total, nfinal); if (rc) return rc; }
-    base = nbase; blen = nblen; final = nfinal;
+    if (!done && !ahead) { rc = prefix_launch(ctx, sp, rin + w.base, w); if (rc) return rc; }
   }
-  CK(cudaEventRecord(ctx->ev[1], s));
+  CK(cudaEventRecord(ctx->ev_k1, s));
   CK(cudaStreamSynchronize(s));
-  *inout_n_descs = nd;
+  float kernel_ms = 0;
+  CK(cudaEventElapsedTime(&kernel_ms, ctx->ev_k0, ctx->ev_k1));
+  *inout_n_descs = t.n;
   ctx->resident_out = out_used;
-  int worst = 0;
-  if (result) {
-    memset(result, 0, sizeof *result);
-    result->n_subblocks = nd; result->n_batches = nb; result->wr_overlap = (int32_t)first; result->kernel_launches = ctx->launches;
-    result->out_used = out_used;
-    CK(cudaEventElapsedTime(&result->kernel_ms, ctx->ev[0], ctx->ev[1]));
-    for (u32 i = 0; i < nd; ++i) { result->bytes_in += descs[i].bytes_consumed; result->bytes_out += descs[i].out_len; }
-  }
-  for (u32 i = 0; i < nd; ++i) if (descs[i].status < worst) worst = descs[i].status;
-  if (worst) ctx->err = std::string("a subblock failed: ") + phy_strerror(worst);
-  return worst;
+  return walk_result(ctx, w, t, out_used, kernel_ms, 0, 0, result);
 }
 
 extern "C" int phy_download(phy_ctx *ctx, uint8_t *out, uint64_t out_cap, uint64_t *out_len) {
@@ -732,21 +772,17 @@ extern "C" int phy_download(phy_ctx *ctx, uint8_t *out, uint64_t out_cap, uint64
   return PHY_OK;
 }
 
-/* second buffers, copy streams and events of the pipelined region call */
-static int pipeline_init(phy_ctx *ctx) {
-  if (ctx->s_in) return PHY_OK;
-  CK(cudaStreamCreateWithFlags(&ctx->s_in, cudaStreamNonBlocking));
-  CK(cudaStreamCreateWithFlags(&ctx->s_out, cudaStreamNonBlocking));
+/* Copy streams, events and second buffers of the pipelined region call; the second input buffer is only needed for regions
+ * of several batches. */
+static int copy_init(phy_ctx *ctx, bool second_input) {
+  CK(ctx->s_in.ensure(0)); /* default priority */
+  CK(ctx->s_out.ensure(0));
   for (int i = 0; i < 2; ++i) {
-    CK(cudaEventCreate(&ctx->ev_in[i]));
-    CK(cudaEventCreateWithFlags(&ctx->ev_c[i], cudaEventDisableTiming));
-    CK(cudaEventCreate(&ctx->ev_out[i]));
-    CK(cudaEventCreate(&ctx->ev_h0[i]));
-    CK(cudaEventCreate(&ctx->ev_d0[i]));
+    for (Event *e : {&ctx->ev_in[i], &ctx->ev_out[i], &ctx->ev_h0[i], &ctx->ev_d0[i]}) CK(e->ensure(cudaEventDefault));
+    CK(ctx->ev_c[i].ensure(cudaEventDisableTiming));
   }
-  CK(cudaHostAlloc(&ctx->h_nl, 64, cudaHostAllocDefault));
-  memset(ctx->h_nl, 0, 64);
-  ctx->h_nl[0] = '\n';
+  if (second_input) CK(ctx->in2.ensure(ctx->max_batch + 4096, true));
+  CK(ctx->out2.ensure(ctx->out_cap + 64));
   return PHY_OK;
 }
 
@@ -754,9 +790,6 @@ static int pipeline_init(phy_ctx *ctx) {
 /* The caller's region is not in memory: reader threads pull it chunk by chunk through the caller's read callback into a
  * ring of pinned staging slots, the uploads consume the chunks in order, payloads come back into two pinned output slots and
  * are handed to the caller's emit callback one batch behind the kernels. */
-static const u64 RING_CHUNK = 16ull << 20;
-static const int RING_SLOTS = 8;
-static const int HOUT_SLOTS = 4; /* pinned payload slots: one being filled by the copy engine, the others with the emitter thread */
 struct StreamIO {
   phy_read_fn read = nullptr; void *ruser = nullptr; phy_emit_fn emit = nullptr; void *euser = nullptr;
   phy_ctx *ctx = nullptr; u64 region_len = 0, nchunks = 0;
@@ -863,50 +896,37 @@ static int compress_region_impl(phy_ctx *ctx, const uint8_t *region, uint64_t re
   CK(cudaSetDevice(ctx->device));
   /* `wait` (streamed variant): region[0, upto) is only valid after wait(user, upto) has returned */
   auto need = [&](u64 upto) { if (wait) wait(wait_user, upto < region_len ? upto : region_len); };
-  PlanState st;
-  if (params && params->rank != 0) need(1u << 20); /* the '@' heuristic looks at the head of the region */
+  if (params && params->rank != 0) need(HEAD_BYTES);
   const uint8_t *head = region;
   if (io) { /* streamed I/O: the head of the region is the head of chunk 0 */
     head = io->chunk(0);
     if (!head) { ctx->err = "reading the region failed"; return PHY_ERR_ARG; }
   }
-  int rc = init_plan(ctx, head, region_len, params, 0, false, st);
+  Walk w;
+  int rc = walk_init(ctx, head, region_len, params, w);
   if (rc) return rc;
-  const u32 first = st.rec_start;
-  *ctx->h_state = st;
-  ctx->launches = 0;
   cudaStream_t s = ctx->stream;
-  CK(cudaMemcpyAsync(ctx->plan_state, ctx->h_state, sizeof(PlanState), cudaMemcpyHostToDevice, s));
   CK(cudaStreamSynchronize(s));
   const bool multi = region_len > ctx->max_batch;
-  rc = pipeline_init(ctx);
+  rc = copy_init(ctx, multi);
   if (rc) return rc;
-  if (multi && !ctx->in2) { CK(cudaMalloc(&ctx->in2, ctx->max_batch + 4096)); CK(cudaMemset(ctx->in2, 0, ctx->max_batch + 4096)); }
-  if (!ctx->out2) CK(cudaMalloc(&ctx->out2, ctx->out_cap + 64));
   u8 *inb[2] = {ctx->in, multi ? ctx->in2 : ctx->in}, *outb[2] = {ctx->out, ctx->out2};
-  const u64 back = batch_back(ctx, params);
-  if (multi && ctx->max_batch < 2 * back + 4096) { ctx->err = "max_batch_bytes is too small for the window size"; return PHY_ERR_CAPACITY; }
   std::vector<phy_subblock_desc> batch_descs; /* streamed I/O: descriptors of one batch at a time */
   if (io) { batch_descs.resize(ctx->max_sb); descs = batch_descs.data(); }
   const u32 cap_descs = io ? ctx->max_sb : *inout_n_descs;
-  u32 nd = 0, nb = 0, nup = 0, nd_total = 0;
-  u64 bytes_in_total = 0, bytes_out_total = 0;
-  u64 out_used = 0, next_pos = 0;
+  Tally t;
+  u32 nd = 0;
+  u64 out_used = 0;
   float k_ms = 0, h2d_ms = 0, d2h_ms = 0;
-  int worst = 0;
-  bool patch_nl = false; /* decided when the final batch is uploaded (the region's last byte must be there) */
 
   /* enqueue the upload of the batch that starts at `base` into input buffer `slot` (stream s_in).  Bytes that the
    * previous upload already brought to the device (the tail of the other buffer: consecutive batches overlap by one
    * window + slack) are copied device-to-device instead of crossing PCIe a second time. */
   u64 up_base = 0, up_blen = 0; int up_slot = -1; /* last upload issued on s_in */
   bool up_timed[2] = {false, false};
-  auto upload = [&](u64 base, int slot, u64 &blen, bool &final, u64 &len) -> int {
-    blen = region_len - base;
-    if (blen > ctx->max_batch) blen = ctx->max_batch;
-    final = base + blen == region_len;
-    len = blen;
-    if (up_timed[slot]) { float t; CK(cudaEventSynchronize(ctx->ev_in[slot])); CK(cudaEventElapsedTime(&t, ctx->ev_h0[slot], ctx->ev_in[slot])); h2d_ms += t; up_timed[slot] = false; }
+  auto upload = [&](u64 base, int slot) -> int {
+    const u64 blen = w.len_at(base);
+    if (up_timed[slot]) { float ms; CK(cudaEventSynchronize(ctx->ev_in[slot])); CK(cudaEventElapsedTime(&ms, ctx->ev_h0[slot], ctx->ev_in[slot])); h2d_ms += ms; up_timed[slot] = false; }
     CK(cudaEventRecord(ctx->ev_h0[slot], ctx->s_in));
     u64 carry = 0;
     if (up_slot >= 0 && up_slot != slot && base >= up_base && base < up_base + up_blen) {
@@ -941,16 +961,13 @@ static int compress_region_impl(phy_ctx *ctx, const uint8_t *region, uint64_t re
       if (base + o + n == region_len) last_byte = src[n - 1];
       o += n;
     }
-    if (final) patch_nl = st.is_last && last_byte != '\n';
-    if (final && patch_nl) { /* last rank whose file does not end in a newline: the reference's arithmetic still places the
-                              * next record start one byte past the end; a virtual newline gives the splitter the same view */
-      CK(cudaMemcpyAsync(inb[slot] + blen, ctx->h_nl, 64, cudaMemcpyHostToDevice, ctx->s_in));
-      len += 1;
-    } else {
-      CK(cudaMemsetAsync(inb[slot] + blen, 0, 64, ctx->s_in));
+    CK(cudaMemsetAsync(inb[slot] + blen, 0, 64, ctx->s_in)); /* zero padding: vector loads may run past the end */
+    if (base + blen == region_len && w.st.is_last && last_byte != '\n') { /* see Walk::nl */
+      w.nl = true;
+      CK(cudaMemsetAsync(inb[slot] + blen, '\n', 1, ctx->s_in));
     }
     CK(cudaEventRecord(ctx->ev_in[slot], ctx->s_in));
-    up_timed[slot] = true; ++nup;
+    up_timed[slot] = true;
     up_base = base; up_blen = blen; up_slot = slot;
     return PHY_OK;
   };
@@ -960,36 +977,32 @@ static int compress_region_impl(phy_ctx *ctx, const uint8_t *region, uint64_t re
    * where the window chain stops here).  Output buffers alternate every round: the payloads of round r leave for the
    * host on s_out while round r + 1 runs. */
   int cur = 0, oslot = 0;
-  u64 base = 0, blen = 0, len = 0;
-  bool final = false;
-  rc = upload(0, cur, blen, final, len);
+  rc = upload(0, cur);
   if (rc) return rc;
-  u64 nbase = 0, nblen = 0, nlen = 0;
-  bool nfinal = false, have_next = false, done = false;
+  bool have_next = false, done = false;
   bool have_d2h[2] = {false, false};
   auto speculate = [&]() -> int { /* the kernels of the batch before the previous one have left the other input buffer (the host synchronised on them) */
-    if (final || have_next || !multi) return PHY_OK;
-    nbase = (base + blen - back) & ~(u64)255;
-    int r = upload(nbase, cur ^ 1, nblen, nfinal, nlen);
+    if (w.final || have_next) return PHY_OK;
+    int r = upload(w.candidate(), cur ^ 1);
     have_next = r == PHY_OK;
     return r;
   };
+  const bool late = wait != nullptr || io != nullptr; /* bytes may not be there yet: waiting for them must not hold this batch's kernels back */
   while (!done) {
-    const bool late = wait != nullptr || io != nullptr; /* bytes may not be there yet: waiting for them must not hold this batch's kernels back */
     if (!late) { rc = speculate(); if (rc) return rc; } /* region bytes are all there: the next upload is queued before this batch's kernels */
     CK(cudaStreamWaitEvent(s, ctx->ev_in[cur], 0));
     if (have_d2h[oslot]) CK(cudaStreamWaitEvent(s, ctx->ev_out[oslot], 0)); /* the payloads of the round before the previous one have left that buffer */
-    CK(cudaEventRecord(ctx->ev[1], s));
-    const u32 start_pos = (u32)(next_pos - base) + (nb == 0 ? first : 0u);
-    rc = run_batch(ctx, inb[cur], outb[oslot], ctx->out_cap, (u32)len, start_pos, (i64)base, (i64)region_len, final);
+    CK(cudaEventRecord(ctx->ev_k0, s));
+    rc = run_batch(ctx, inb[cur], outb[oslot], ctx->out_cap, w);
     if (rc) return rc;
-    CK(cudaEventRecord(ctx->ev[2], s));
+    CK(cudaEventRecord(ctx->ev_k1, s));
     CK(cudaEventRecord(ctx->ev_c[oslot], s));
     if (late) { rc = speculate(); if (rc) return rc; }
     CK(cudaStreamSynchronize(s));
     const u32 S = ctx->last_S;
-    const PlanState hs = *ctx->h_state;
-    if (hs.status) { ctx->err = std::string("window chaining failed: ") + phy_strerror(hs.status); return hs.status; }
+    bool move;
+    rc = w.after(ctx, *ctx->h_state, S, done, move);
+    if (rc) return rc;
     if (io) { nd = 0; out_used = 0; } /* every batch goes to its own pinned output slot and descriptor list */
     if (nd + S > cap_descs) { ctx->err = "descriptor array too small"; return PHY_ERR_CAPACITY; }
     const u64 tot = S ? ctx->h_hdr->total_out : 0;
@@ -997,7 +1010,7 @@ static int compress_region_impl(phy_ctx *ctx, const uint8_t *region, uint64_t re
     int hslot = -1;
     if (io) { hslot = io->acquire_hslot(); if (hslot < 0) { ctx->err = "the emit callback stopped the call"; return PHY_ERR_ARG; } }
     uint8_t *hdst = io ? ctx->hout[hslot] : out + out_used;
-    if (have_d2h[oslot]) { float t; CK(cudaEventElapsedTime(&t, ctx->ev_d0[oslot], ctx->ev_out[oslot])); d2h_ms += t; have_d2h[oslot] = false; }
+    if (have_d2h[oslot]) { float ms; CK(cudaEventElapsedTime(&ms, ctx->ev_d0[oslot], ctx->ev_out[oslot])); d2h_ms += ms; have_d2h[oslot] = false; }
     CK(cudaStreamWaitEvent(ctx->s_out, ctx->ev_c[oslot], 0));
     CK(cudaEventRecord(ctx->ev_d0[oslot], ctx->s_out));
     if (tot) CK(cudaMemcpyAsync(hdst, outb[oslot], tot, cudaMemcpyDeviceToHost, ctx->s_out));
@@ -1005,56 +1018,34 @@ static int compress_region_impl(phy_ctx *ctx, const uint8_t *region, uint64_t re
     if (io) CK(cudaEventRecord(ctx->ev_hout[hslot], ctx->s_out));
     have_d2h[oslot] = true;
     fill_descs(ctx, S, out_used, descs + nd);
-    for (u32 i = 0; i < S; ++i) { bytes_in_total += descs[nd + i].bytes_consumed; bytes_out_total += descs[nd + i].out_len; if (descs[nd + i].status < worst) worst = descs[nd + i].status; }
-    nd_total += S;
+    t.add(descs + nd, S);
     if (io) io->push_item(descs, S, hslot); /* the emitter thread hands the batch to the caller once its payloads have arrived */
-    float t;
-    CK(cudaEventElapsedTime(&t, ctx->ev[1], ctx->ev[2])); k_ms += t;
-    nd += S; out_used += tot; ++nb; oslot ^= 1;
-    done = hs.done != 0;
-    if (!done) {
-      const u64 stopped = (u64)hs.bytes_read;
-      if (S == 0 && stopped == next_pos && (final || stopped < ((base + blen - back) & ~(u64)255))) {
-        ctx->err = final ? "region exhausted before the working region was covered" : "a window does not fit one batch (raise max_batch_bytes)";
-        return final ? PHY_ERR_MALFORMED : PHY_ERR_CAPACITY;
-      }
-      next_pos = stopped;
-      if (have_next && next_pos >= nbase) { /* on to the next batch */
-        cur ^= 1; base = nbase; blen = nblen; len = nlen; final = nfinal; have_next = false;
-      } /* else: the chain stopped early because the batch's subblock capacity was used up; the next round continues in the same bytes */
-    }
+    float ms;
+    CK(cudaEventElapsedTime(&ms, ctx->ev_k0, ctx->ev_k1)); k_ms += ms;
+    nd += S; out_used += tot; oslot ^= 1;
+    if (move) { cur ^= 1; w.place(w.candidate()); have_next = false; } /* else the next round continues in the same bytes */
   }
   CK(cudaStreamSynchronize(ctx->s_in));
   CK(cudaStreamSynchronize(ctx->s_out));
   for (int i = 0; i < 2; ++i) {
-    if (have_d2h[i]) { float t; CK(cudaEventElapsedTime(&t, ctx->ev_d0[i], ctx->ev_out[i])); d2h_ms += t; }
-    if (up_timed[i]) { float t; CK(cudaEventElapsedTime(&t, ctx->ev_h0[i], ctx->ev_in[i])); h2d_ms += t; }
+    float ms;
+    if (have_d2h[i]) { CK(cudaEventElapsedTime(&ms, ctx->ev_d0[i], ctx->ev_out[i])); d2h_ms += ms; }
+    if (up_timed[i]) { CK(cudaEventElapsedTime(&ms, ctx->ev_h0[i], ctx->ev_in[i])); h2d_ms += ms; }
   }
   if (io && !io->finish_emit()) { ctx->err = "the emit callback stopped the call"; return PHY_ERR_ARG; }
-  if (inout_n_descs) *inout_n_descs = io ? nd_total : nd;
-  if (result) {
-    memset(result, 0, sizeof *result);
-    result->n_subblocks = nd_total; result->n_batches = nb; result->wr_overlap = (int32_t)first; result->kernel_launches = ctx->launches;
-    result->kernel_ms = k_ms; result->h2d_ms = h2d_ms; result->d2h_ms = d2h_ms; result->out_used = io ? bytes_out_total : out_used;
-    result->bytes_in = bytes_in_total; result->bytes_out = bytes_out_total;
-  }
-  if (worst) ctx->err = std::string("a subblock failed: ") + phy_strerror(worst);
-  return worst;
+  if (inout_n_descs) *inout_n_descs = t.n;
+  return walk_result(ctx, w, t, io ? t.bytes_out : out_used, k_ms, h2d_ms, d2h_ms, result);
 }
 
 extern "C" int phy_stream_prepare(phy_ctx *ctx) {
   if (!ctx) return PHY_ERR_ARG;
   CK(cudaSetDevice(ctx->device));
-  int rc = pipeline_init(ctx);
+  int rc = copy_init(ctx, true);
   if (rc) return rc;
-  if (!ctx->ring) {
-    CK(cudaHostAlloc(&ctx->ring, RING_CHUNK * RING_SLOTS, cudaHostAllocDefault));
-    for (int i = 0; i < HOUT_SLOTS; ++i) CK(cudaHostAlloc(&ctx->hout[i], ctx->out_cap + 64, cudaHostAllocDefault));
-    for (int i = 0; i < RING_SLOTS; ++i) CK(cudaEventCreateWithFlags(&ctx->ev_ring[i], cudaEventDisableTiming));
-    for (int i = 0; i < HOUT_SLOTS; ++i) CK(cudaEventCreateWithFlags(&ctx->ev_hout[i], cudaEventDisableTiming));
-  }
-  if (!ctx->in2) { CK(cudaMalloc(&ctx->in2, ctx->max_batch + 4096)); CK(cudaMemset(ctx->in2, 0, ctx->max_batch + 4096)); }
-  if (!ctx->out2) CK(cudaMalloc(&ctx->out2, ctx->out_cap + 64));
+  CK(ctx->ring.ensure(RING_CHUNK * RING_SLOTS));
+  for (auto &h : ctx->hout) CK(h.ensure(ctx->out_cap + 64));
+  for (auto &e : ctx->ev_ring) CK(e.ensure(cudaEventDisableTiming));
+  for (auto &e : ctx->ev_hout) CK(e.ensure(cudaEventDisableTiming));
   return PHY_OK;
 }
 
@@ -1066,9 +1057,7 @@ extern "C" int phy_compress_stream(phy_ctx *ctx, uint64_t region_len, const phy_
   StreamIO io;
   io.read = read; io.ruser = read_user; io.emit = emit; io.euser = emit_user; io.ctx = ctx; io.region_len = region_len;
   io.nchunks = (region_len + RING_CHUNK - 1) / RING_CHUNK;
-  static const int nreaders_env = getenv("PHY_READERS") ? atoi(getenv("PHY_READERS")) : 6;
-  const int nreaders = nreaders_env < 1 ? 1 : nreaders_env > RING_SLOTS ? RING_SLOTS : nreaders_env;
-  for (int t = 0; t < nreaders; ++t) io.readers.emplace_back([&io, t, nreaders] { io.reader_main(t, nreaders); });
+  for (int t = 0; t < READERS; ++t) io.readers.emplace_back([&io, t] { io.reader_main(t, READERS); });
   io.emitter = std::thread([&io] { io.emitter_main(); });
   rc = compress_region_impl(ctx, nullptr, region_len, params, nullptr, nullptr, nullptr, 0, nullptr, nullptr, result, &io);
   io.shutdown();
@@ -1091,7 +1080,7 @@ extern "C" int phy_compress_region_streamed(phy_ctx *ctx, const uint8_t *region,
 extern "C" int phy_profile(phy_ctx *ctx, int enable) {
   if (!ctx) return PHY_ERR_ARG;
   CK(cudaSetDevice(ctx->device));
-  if (enable && !ctx->pev[0]) for (auto &e : ctx->pev) CK(cudaEventCreate(&e));
+  if (enable) for (auto &e : ctx->pev) CK(e.ensure(cudaEventDefault));
   ctx->profile = enable != 0;
   for (auto &m : ctx->pms) m = 0;
   ctx->pcount = 0;
