@@ -29,7 +29,11 @@ enum {
   PHY_ERR_FIELDS = -2,      /* separator count differs between titles (reference: warning then UB, :417-421) */
   PHY_ERR_COLORSPACE = -3,  /* colour-space reads (phyNGSC.cpp:473-547) are not implemented                  */
   PHY_ERR_UNSUPPORTED = -4, /* outside the reference's defined domain: >32 title fields, token >512 B,
-                               field max_len == 128 (Q11), Huffman code > 32 bits, read > 32767, NUL bytes    */
+                               field max_len == 128 (Q11), Huffman code > 32 bits, NUL bytes; or beyond the
+                               kernels' limits: a read of 512 bases or more (the per-position quality table
+                               has 512 rows) fails its subblock, and so do 32 records of more than 24 KiB
+                               whose packed quality tables exceed 24 KiB (e.g. 511 bp reads with more than
+                               24 quality symbols)                                                            */
   PHY_ERR_CAPACITY = -5,    /* a ctx buffer (batch bytes, records, arena, output) is too small               */
   PHY_ERR_CUDA = -6,        /* CUDA runtime error / no device; see phy_last_error()                          */
   PHY_ERR_ARG = -7

@@ -552,10 +552,14 @@ static int run_body(phy_ctx *ctx, u8 *out, u64 out_cap) {
     /* Shared memory for the packed quality tables: (longest read + 1) x alphabet x 2 bytes.  The alphabet size is known
      * on the device only; the first batch of a context waits for the readback, later batches reserve room for the
      * alphabet the previous batch had plus eight symbols, so the GPU never waits for the host here (a subblock whose
-     * tables outgrow the reservation reads them from global memory instead -- slower, same bytes). */
+     * tables outgrow the reservation reads them from global memory instead -- slower, same bytes).  While the previous
+     * alphabet's own tables fit PK_SMEM_MAX, the reservation is cut to PK_SMEM_MAX: the eight spare symbols must not push
+     * tables that fit out of shared memory (long reads would lose the single-walk kernels on every batch after the first). */
     u32 pk;
-    if (nq_hint) pk = ((H.max_len + 1) * (nq_hint + 8 > 256 ? 256u : nq_hint + 8) * 2u + 15u) & ~15u;
-    else { CK(cudaEventSynchronize(ctx->ev_rb[g])); pk = (ctx->h_hdr_g[g].max_pk_bytes + 15u) & ~15u; }
+    if (nq_hint) {
+      pk = ((H.max_len + 1) * (nq_hint + 8 > 256 ? 256u : nq_hint + 8) * 2u + 15u) & ~15u;
+      if (pk > PK_SMEM_MAX && (((H.max_len + 1) * nq_hint * 2u + 15u) & ~15u) <= PK_SMEM_MAX) pk = PK_SMEM_MAX;
+    } else { CK(cudaEventSynchronize(ctx->ev_rb[g])); pk = (ctx->h_hdr_g[g].max_pk_bytes + 15u) & ~15u; }
     e.pk_bytes = pk <= PK_SMEM_MAX ? pk : 0u; /* larger tables stay in global memory (L1) */
     k_huff<<<dim3(HUFF_LARGE + 32, Sg), HUFF_WARPS * 32, HUFF_SMEM, gs>>>(e); GMARK();
     /* single-walk encoder: slots, then title + info and quality + DNA of every task into the temporary buffer */

@@ -2,6 +2,7 @@
 // phyngsc_b200/csrc/phy_core.cuh together serially on the CPU so that tokeniser, classification, Huffman,
 // header layout, walkers and bit sinks can be checked against the oracle without a GPU.  It is not a
 // fallback: nothing in the product links or loads it.
+#include <stddef.h>
 #include <stdlib.h>
 #include <string.h>
 
@@ -383,6 +384,15 @@ extern "C" int mirror_compress_window(const u8 *b, u64 readable, i64 rsize, u32 
 extern "C" int mirror_compress_window_fast(const u8 *b, u64 readable, i64 rsize, u32 rec_start, i32 overlap, u32 cap,
                                            u8 *out, u32 out_cap, u32 *sec_len, u32 *n_records, u64 *bytes_consumed, u32 lanes_per_record) {
   return mirror_window(b, readable, rsize, rec_start, overlap, cap, out, out_cap, sec_len, n_records, bytes_consumed, lanes_per_record);
+}
+
+/* where the encoder-path fields sit in SbClass, for tests that decode the GPU's per-subblock records
+ * (phy_debug_read(ctx, "cls", ...)): sizeof, then the byte offsets of status, fast, qpk_esc, max_qlen, nq */
+extern "C" u32 mirror_sbclass_layout(u32 *v, u32 n) {
+  const u32 w[6] = {(u32)sizeof(SbClass), (u32)offsetof(SbClass, status), (u32)offsetof(SbClass, fast), (u32)offsetof(SbClass, qpk_esc),
+                    (u32)offsetof(SbClass, max_qlen), (u32)offsetof(SbClass, nq)};
+  for (u32 i = 0; i < n && i < 6; ++i) v[i] = w[i];
+  return 6;
 }
 
 extern "C" u32 mirror_huffman(const u32 *freq, u32 n, u64 *cl, u8 *tree) {

@@ -2,34 +2,17 @@
 tests/mirror/mirror.cpp and checked against the oracle: tokeniser, classification, Huffman build and
 serialisation, header layout, stream walkers and bit sinks.  The CUDA kernels call the same functions."""
 import ctypes as C
-import os
-import subprocess
 
 import numpy as np
 import pytest
 
+import gpu_cases
 from phyngsc_b200 import synth
-
-HERE = os.path.dirname(os.path.abspath(__file__))
-SRC = os.path.join(HERE, "mirror", "mirror.cpp")
-LIB = os.path.join(HERE, "mirror", "libmirror.so")
-CORE = os.path.join(HERE, "..", "phyngsc_b200", "csrc", "phy_core.cuh")
-FAST = os.path.join(HERE, "..", "phyngsc_b200", "csrc", "phy_fast.cuh")
 
 
 @pytest.fixture(scope="module")
 def mirror():
-    if not os.path.exists(LIB) or os.path.getmtime(LIB) < max(os.path.getmtime(SRC), os.path.getmtime(CORE), os.path.getmtime(FAST)):
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-x", "c++", "-fPIC", "-shared", "-o", LIB, SRC])
-    L = C.CDLL(LIB)
-    L.mirror_compress_window.restype = C.c_int
-    L.mirror_compress_window.argtypes = [C.c_void_p, C.c_uint64, C.c_int64, C.c_uint32, C.c_int32, C.c_uint32, C.c_void_p,
-                                         C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]
-    L.mirror_compress_window_fast.restype = C.c_int
-    L.mirror_compress_window_fast.argtypes = L.mirror_compress_window.argtypes + [C.c_uint32]
-    L.mirror_huffman.restype = C.c_uint32
-    L.mirror_huffman.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]
-    return L
+    return gpu_cases.mirror()
 
 
 @pytest.mark.parametrize("shape", ["36bp", "100bp", "100bp_huffdna", "150bp_paired", "var50_205", "var50_250", "title_stress",
